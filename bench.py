@@ -16,12 +16,12 @@ block size 4096, LPC order 8, Rice parameter 4, mid/side.  One *step* = one pass
            (default): `--inflight` units per rank; `--scaling strong`: a fixed corpus of `--units`
            units split over the ranks.  A lone 1024-frame batch is latency-bound by the serial LPC
            recurrence (SURVEY.md §7.3-3) and the sequential Rice walk; its figure is reported next to
-           it as `single_batch`.  A step takes ~15 us, so `--steps K` alone would be a sub-millisecond
-           window: the timed region is `repeats` x K steps issued back to back (no drain in between;
-           `repeats` is chosen so that the region holds >= --min-steps steps), it is measured
-           `--regions` times and the median region is reported; ms_per_step = region / (repeats * K).
-           Every batch's CUDA graph is instantiated when the batch is created and every batch is
-           decoded once before anything is timed, whatever --warmup says.
+           it as `single_batch`.  The timed region is `--steps K` steps issued back to back (no drain in
+           between; `--scaling strong`: K steps of the whole corpus, each rank running those of its own
+           units); ms_per_step = region / K.  A step takes ~15 us, so K of a few thousand is needed for a
+           window of tens of milliseconds.  Every batch's CUDA graph is instantiated when the batch is
+           created, and `--warmup W` untimed steps precede the region, never fewer than one per unit.
+           `--dump-outputs DIR` then writes what the last timed step computed (`dump_outputs`).
   e2e    — same metric through the public host-buffer call (`clx_decode_frames`): per step the
            compressed frames go pinned-host -> device and the full planar i32 PCM comes back.  The call
            is synchronous; `--e2e-callers` host threads (default 2, each with its own context and pinned
@@ -54,8 +54,10 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
+sys.dont_write_bytecode = True  # the tree may be read-only; the benchmark writes nothing into it
 
 METRIC = "Msamples/s decoded (bit-exact)"
+DUMP_LIMIT_BYTES = 64 * 10**6
 
 # frames per unit (one device-resident batch) of each workload, and units of the whole corpus (strong scaling)
 UNIT_FRAMES = {"c2": 1024, "c2-indep": 1024, "c3": 8192, "c4": 1100, "c5": 256}
@@ -216,6 +218,34 @@ def unit_config(synth, workload, unit_index, frames=None):
     return cfg
 
 
+def dump_outputs(dirpath, batch):
+    """Writes what a caller of the device-resident path gets back from `batch` (clx_batch_read) as .npy files, so
+    that two builds can be compared output for output:
+      pcm.npy        decoded samples, each frame planar as claxon's Block, frames back to back (the alignment
+                     padding between frames in the output buffer is left out); float32 when every sample fits
+                     its 24-bit significand, float64 otherwise
+      pcm_frames.npy the frame index of each frame in pcm.npy, in order
+      status.npy, consumed.npy  every frame's result
+    When all samples would not fit DUMP_LIMIT_BYTES in all, pcm.npy holds a fixed, seeded selection of whole
+    frames."""
+    out, res = batch.read()
+    d = batch.descs
+    offs = d["out_offset"].astype(np.int64)
+    lens = d["n_channels"].astype(np.int64) * d["block_size"].astype(np.int64)
+    peak = max((int(np.abs(out[o:o + n].astype(np.int64)).max(initial=0)) for o, n in zip(offs, lens)), default=0)
+    dtype = np.dtype(np.float32 if peak <= 2**24 else np.float64)
+    fixed = 3 * 8 * d.size + 4 * 4096  # the per-frame arrays and the .npy headers
+    sel = np.arange(d.size)
+    if int(lens.sum()) * dtype.itemsize + fixed > DUMP_LIMIT_BYTES:
+        order = np.random.default_rng(0).permutation(d.size)
+        sel = np.sort(order[np.cumsum(lens[order]) * dtype.itemsize + fixed <= DUMP_LIMIT_BYTES])
+    pcm = np.concatenate([out[offs[i]:offs[i] + lens[i]] for i in sel] or [np.zeros(0, np.int32)])
+    os.makedirs(dirpath, exist_ok=True)
+    for name, a in (("pcm", pcm.astype(dtype)), ("pcm_frames", sel.astype(np.float64)),
+                    ("status", res["status"].astype(np.float64)), ("consumed", res["consumed"].astype(np.float64))):
+        np.save(os.path.join(dirpath, name + ".npy"), a)
+
+
 class Job:
     """This rank's share of a list of units, resident on the device."""
 
@@ -249,10 +279,11 @@ class Job:
                 return False
         return True
 
-    def steady(self, ctx, steps, streams, regions, sync=None):
-        """`regions` timed regions of `steps` steps each (round-robin over this rank's units); device ms each."""
+    def steady(self, ctx, steps, streams, regions, sync=None, warmup=0):
+        """`warmup` untimed steps (every batch once, at least), then `regions` timed regions of `steps` steps each
+        (round-robin over this rank's units); device ms each."""
         n = len(self.batches)
-        ctx.run_steps(self.batches, max(n, 3), streams)  # every batch once, at least
+        ctx.run_steps(self.batches, max(n, 3, warmup), streams)
         out = []
         for _ in range(max(1, regions)):
             if sync:
@@ -295,10 +326,8 @@ def short_line(cb, synth, ctx, workload, n_units, streams, min_ms=40.0):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
-    ap.add_argument("--min-steps", type=int, default=4000, help="the timed region holds at least this many steps (repeats x steps)")
-    ap.add_argument("--regions", type=int, default=3, help="timed regions; the median is reported")
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=4000, help="steps in the timed region")
+    ap.add_argument("--warmup", type=int, default=5, help="untimed steps before it (at least one per unit)")
     ap.add_argument("--impl", default="claxon_b200", choices=["claxon_b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(UNIT_FRAMES))
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
@@ -310,7 +339,13 @@ def main():
     ap.add_argument("--e2e-callers", type=int, default=2)
     ap.add_argument("--cpu-seconds", type=float, default=3.0)
     ap.add_argument("--no-extra", action="store_true", help="skip the short c3 / c4 / c5 lines at N=1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step decoded to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "claxon_b200":
+        ap.error("--dump-outputs writes the outputs of the device path (--impl claxon_b200)")
 
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     # more hardware work queues than the default 8, so that the batches in flight really overlap
@@ -431,26 +466,28 @@ def main():
 
     # ---- steady state
     if args.scaling == "weak":
-        repeats = max(1, -(-args.min_steps // max(1, args.steps)))
-        my_steps = repeats * args.steps        # per rank; the job's steps are world x that
+        my_steps = args.steps                  # per rank; the job's steps are world x that
         timed_steps = my_steps * world
-    else:  # a step = one unit of the corpus; a region = `repeats` passes over the whole corpus
-        repeats = max(1, -(-max(args.min_steps, args.steps) // n_units))
-        my_steps = repeats * n_mine
-        timed_steps = repeats * n_units
+    else:  # a step = one unit of the corpus; step i decodes unit i % n_units, on the rank that holds it
+        full, rem = divmod(args.steps, n_units)
+        my_steps = full * n_mine + max(0, min(hi, rem) - lo)
+        timed_steps = args.steps
+    warm_steps = max(n_mine, 3, args.warmup)
     sampler = ClockSampler(local)
     sampler.start()
     launches0 = ctx.launch_count
     t_wall0 = time.time()
-    regions = [max_over_ranks(r) for r in (job.steady(ctx, my_steps, args.streams, args.regions, barrier) if n_mine
-                                            else [0.0] * max(1, args.regions))]
+    regions = [max_over_ranks(r) for r in (job.steady(ctx, my_steps, args.streams, 1, barrier, warm_steps) if n_mine
+                                            else [0.0])]
     t_wall1 = time.time()
     launches_all = ctx.launch_count - launches0
     barrier()
     clocks = sampler.stop(t_wall0, t_wall1)
     ms = float(np.median(regions))
     my_samples, my_alg = job.per_steps(my_steps) if n_mine else (0, 0)
-    gpu_launches = int(round(launches_all * my_steps / (my_steps * max(1, args.regions) + max(n_mine, 3)))) if n_mine else 0
+    gpu_launches = int(round(launches_all * my_steps / (my_steps + warm_steps))) if n_mine else 0
+    if args.dump_outputs and rank == 0 and my_steps:
+        dump_outputs(args.dump_outputs, job.batches[(my_steps - 1) % n_mine])
     tot_samples, tot_alg = sum_over_ranks(my_samples), sum_over_ranks(my_alg)
     value = tot_samples / (ms / 1e3) / 1e6
     peak, peak_src = measured_peak_gbs()
@@ -569,7 +606,7 @@ def main():
         e2e_main = e2e.get("e2e", {"value": None, "unit": "Msamples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0})
         line = {
             "metric": METRIC, "value": value, "unit": "Msamples/s", "n_gpus": world, "steps": args.steps,
-            "warmup": max(args.warmup, 3), "ms_per_step": ms / timed_steps, "repeats": repeats, "timed_steps": timed_steps,
+            "warmup": warm_steps, "ms_per_step": ms / timed_steps, "timed_steps": timed_steps,
             "region_ms": regions, "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None,
             "dtype": "int32 samples / int64 accumulate", "data": "synthetic", "config": config, "bit_exact": bool(exact),
             "clocks": clocks, "gpu_launches": gpu_launches,

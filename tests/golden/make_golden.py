@@ -1,10 +1,10 @@
 """Generates tests/golden/fixtures.npz from the reference's own test streams.
 
-Run in the authoring container (needs /root/reference; the GPU box does not have it):
+Run with the test streams of a claxon checkout:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <claxon checkout>/testsamples
 
-For every stream under /root/reference/testsamples (incl. the fuzz corpus) it stores the raw
+For every stream in that directory (incl. the fuzz corpus) it stores the raw
 bytes, the status the oracle reports at open / first failing frame, and — for streams that
 decode — the oracle's planar PCM per frame, which is pinned independently by the STREAMINFO MD5
 (libFLAC's encoder-side digest) wherever the file carries one.  The npz is what the `-m gpu`
@@ -21,15 +21,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from oracle import oracle as O  # noqa: E402
 
-REF = "/root/reference/testsamples"
 
-
-def main():
+def main(ref):
     out = {}
     names = []
-    files = sorted(glob.glob(os.path.join(REF, "*.flac"))) + sorted(glob.glob(os.path.join(REF, "fuzz", "*.flac")))
+    files = sorted(glob.glob(os.path.join(ref, "*.flac"))) + sorted(glob.glob(os.path.join(ref, "fuzz", "*.flac")))
     for path in files:
-        rel = os.path.relpath(path, REF)
+        rel = os.path.relpath(path, ref)
         key = rel.replace("/", "__").replace(".flac", "")
         data = np.fromfile(path, dtype=np.uint8)
         names.append(key)
@@ -77,4 +75,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_golden.py <claxon checkout>/testsamples")
+    main(sys.argv[1])

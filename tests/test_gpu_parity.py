@@ -454,6 +454,33 @@ def test_resident_batch_reports_crc_mismatch():
     c.close()
 
 
+@pytest.mark.parametrize("workload,frames,sampled", [("c2", 64, False), ("c5", 256, True)])
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path, workload, frames, sampled):
+    """bench.py --dump-outputs: 4 timed steps over 2 units end on unit 1, whose PCM and per-frame results are written
+    bit for bit as the generator made them, within 64 MB in all (a c5 unit's 134 MB of samples: a seeded selection
+    of whole frames)."""
+    import subprocess
+    import sys
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--workload", workload, "--inflight", "2", "--streams", "2",
+           "--steps", "4", "--warmup", "1", "--e2e-steps", "1", "--cpu-seconds", "0", "--no-extra",
+           "--frames", str(frames), "--dump-outputs", str(tmp_path)]
+    res = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert res.returncode == 0, res.stderr[-2000:]
+    line = json.loads(res.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 4 and line["timed_steps"] == 4 and line["bit_exact"]
+    cfg = synth.workload_config(workload, frames)
+    cfg.seed += 1000003  # unit 1 (bench.unit_config)
+    b = synth.generate(cfg)
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 * 10**6
+    got = {n: np.load(tmp_path / f"{n}.npy") for n in ("pcm", "pcm_frames", "status", "consumed")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert (got["status"] == 0).all() and np.array_equal(got["consumed"], b.frame_lengths)
+    sel = got["pcm_frames"].astype(np.int64)
+    assert 0 < sel.size <= b.n_frames and sampled == (sel.size < b.n_frames)
+    exp = np.concatenate([b.pcm[int(b.pcm_offsets[i]):int(b.pcm_offsets[i + 1])] for i in sel])
+    assert np.array_equal(got["pcm"].astype(np.int64), exp)
+
+
 def test_constant_frames_through_read_batch(ctx):
     """Digital silence: 14-byte frames that decode to 8192 samples each (ADVICE r1: the batched reader used to size
     its buffer from the remaining BYTES and failed on such streams)."""
