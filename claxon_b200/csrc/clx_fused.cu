@@ -6,7 +6,8 @@
 //      ended), so one lane walks the frame once: subframe headers, warm-up samples and predictor
 //      parameters (src/subframe.rs:29-91, :382-415, :651-701) are parsed and recorded per subframe
 //      together with the bit at which its residual starts; the Rice codes of every channel but the last
-//      are only stepped over (src/subframe.rs:336-348: unary run + k bits), eight per trip.
+//      are only stepped over (src/subframe.rs:336-348: unary run + k bits), in runs of four groups of eight
+//      behind one ring refill.
 //   2. `decode_subframes_kernel` — ONE LANE PER SUBFRAME.  The lane starts at the recorded bit, decodes
 //      its Rice partitions eight codes per trip from a three-word register window over a per-lane
 //      shared-memory ring (src/subframe.rs:236-380) and feeds the residuals, still in registers, to the
@@ -78,7 +79,7 @@ struct DeviceIO {
     }
     // Before a read of at most 16 bytes from bitpos on (a header field, a single code, a window seat): nothing to
     // do if the steady-state refill is far enough ahead — at most max(WAITN, 4) quads behind its front are still
-    // in flight, see prefetch_group() — else a blocking refill.
+    // in flight, see prefetch_group() and prefetch_run() — else a blocking refill.
     __device__ __forceinline__ void ensure_near(uint32_t bitpos) {
         if (fq < (bitpos >> 7) + 2u + (WAITN > 4u ? WAITN : 4u)) ensure(bitpos);
     }
@@ -107,6 +108,34 @@ struct DeviceIO {
             asm volatile("cp.async.wait_group %0;" ::"n"(WAITN) : "memory");
         }
         return true;
+    }
+    // Steady state of the index lane, once per run of groups that consumes at most `quads` quads from bitpos on: the
+    // ring is topped up to RQ quads from the cursor's quad q0 in one commit group.  The run reads quads q0 ..
+    // q0 + quads + 1 (the last one for the window's look-ahead word).  What it reads has landed: every older commit
+    // group has after wait_group 1, and this one's n quads are the newest, from q0 + RQ - n on, beyond the run's
+    // reach while n + quads + 2 <= RQ.  At most max(WAITN, 4) quads are left in flight, as ensure_near() assumes;
+    // a run that has to issue more (a dense stretch, a jump of the cursor) waits for all of them.
+    // The first two copies are predicated, not branched over: a run of light codes (C2: 1.5 quads) needs no more.
+    __device__ __forceinline__ void prefetch_run(uint32_t bitpos, uint32_t quads) {
+        const uint32_t q0 = bitpos >> 7, need = q0 + RQ;
+        if (fq < q0) fq = q0;
+        const uint32_t f0 = fq;
+#pragma unroll
+        for (int i = 0; i < 2; i++) {
+            if (fq < need) { issue(fq); fq++; }
+        }
+        static_assert(2u <= (WAITN > 4u ? WAITN : 4u), "two copies may stay in flight");
+        if (fq < need) {
+            while (fq < need) { issue(fq); fq++; }
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            const uint32_t n = fq - f0;
+            if (n <= (WAITN > 4u ? WAITN : 4u) && n + quads + 2u <= RQ) asm volatile("cp.async.wait_group 1;" ::: "memory");
+            else asm volatile("cp.async.wait_group 0;" ::: "memory");
+        } else {  // n <= 2: the same test, decided at compile time
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            if (quads + 4u <= RQ) asm volatile("cp.async.wait_group 1;" ::: "memory");
+            else asm volatile("cp.async.wait_group 0;" ::: "memory");
+        }
     }
     __device__ __forceinline__ void open(uint32_t ring_addr, uint32_t lane, const uint8_t* bytes, uint64_t buf_bytes,
                                          uint64_t byte_offset) {
@@ -138,7 +167,8 @@ struct DeviceIO {
 // tests pass with it) but 18 % slower than the cp.async ring above — a bulk copy takes uniform-register operands,
 // so the compiler serves 32 lanes with 32 sources through a loop of ~9 instructions per lane, against one LDGSTS
 // for the whole warp (profiles/ab_ring_tma_r02.json vs ab_ring_cpasync_r02.json).  Kept so that the comparison can
-// be repeated; the product library is built without it.
+// be repeated; the product library is built without it.  (Those figures predate the index lane's runs, for which the
+// index ring's chunks went from 128 to 256 bytes; that build compiles but has not been re-run since.)
 // Chunk c of the frame (CHUNK bytes from its 16-byte aligned base) lives in half c & 1.  A half is re-armed
 // only after the cursor has left the chunk it held, so at most one copy per half is ever outstanding and the
 // parity to wait for simply alternates.  Reads past the end of the byte buffer see the buffer's last chunk
@@ -220,6 +250,16 @@ struct TmaIO {
         while (live && cready <= c1) { wait(cready); cready++; }
         return true;
     }
+    // Once per run of groups that consumes at most `quads` quads from bitpos on (the window's look-ahead word
+    // included, it reads up to quad (bitpos >> 7) + quads + 1): needs a CHUNK of at least (quads + 2) * 16 bytes.
+    __device__ __forceinline__ void prefetch_run(uint32_t bitpos, uint32_t quads) {
+        const uint32_t c0 = bitpos / CB, c1 = (((bitpos >> 7) + quads + 1u) << 7) / CB;
+        if (live && creq < c0 + 2u) {
+            if (creq < c0 + 1u) ensure(bitpos);
+            else { request(creq); creq++; }
+        }
+        while (live && cready <= c1) { wait(cready); cready++; }
+    }
     // No copy into this CTA's shared memory may be in flight when the CTA retires.
     __device__ __forceinline__ void close() {
         while (cready < creq) { wait(cready); cready++; }
@@ -250,7 +290,7 @@ struct TmaIO {
 // ---------------------------------------------------------------------------------
 constexpr uint32_t IDX_RQ = 16;
 #ifdef CLX_RING_TMA
-using IndexIO = TmaIO<128>;
+using IndexIO = TmaIO<256>;  // a run of IndexLane::RUN groups reads up to 10 quads: 160 bytes must fit one chunk and the next
 #else
 using IndexIO = DeviceIO<IDX_RQ, 6>;
 #endif
@@ -282,10 +322,11 @@ index_frames_kernel(const uint8_t* __restrict__ bytes, uint64_t buf_bytes, const
         L.rc.ok = true;
     }
     while (__any_sync(0xffffffffu, !L.done())) {
-        // the steady state, a tight loop of its own: every lane of the warp steps over eight codes
-        while (__all_sync(0xffffffffu, L.fast_ready())) L.fast_group();
+        // the steady state, a tight loop of its own: every lane of the warp steps over a run of up to RUN groups of
+        // eight codes (fewer at the end of its partition)
+        while (__all_sync(0xffffffffu, L.fast_ready())) L.run();
         // anything else (headers, partition switches, long codes, lanes that are done): one mixed step
-        if (L.fast_ready()) L.fast_group();
+        if (L.fast_ready()) L.run();
         else if (!L.done()) L.slow_step();
         __syncwarp();
     }

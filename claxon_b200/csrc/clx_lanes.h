@@ -112,6 +112,8 @@ enum : uint32_t { SEQ_SUBFRAME = 0, SEQ_PART = 1, SEQ_RUN = 2, SEQ_DONE = 3 };
 //   uint32_t word(uint32_t wi)            big-endian word `wi` of the frame (relative to its 16-byte aligned base)
 //   void ensure(uint32_t bitpos)          the bits from bitpos on (ring size minus slack) are readable through word()
 //   bool prefetch_group(uint32_t bitpos)  steady-state refill, once per fast group; false: ensure() before reading on
+//   void prefetch_run(uint32_t bitpos, uint32_t quads)   steady-state refill, once per run of groups (skip_run) that
+//                                         consumes at most `quads` 16-byte quads from bitpos on
 //   void seek_next(uint32_t wi), uint32_t next_raw()   sequential word reads, bytes as stored (the register window's refill)
 //   void ensure_near(uint32_t bitpos)     cheap: the next 16 bytes from bitpos are readable (refills, blocking, only if not)
 
@@ -274,32 +276,48 @@ struct RiceCursor {
         }
         return bad;
     }
-    template <bool VALUES>
-    CLX_HD bool codes8_by_cap(int32_t (&e)[8]) {
-        return ncap == 2 ? codes8<2, VALUES>(e) : codes8<1, VALUES>(e);
-    }
     // The group, by the form the partition allows; precondition n_fast != 0.  On failure the cursor is put back
     // and the fast path closed: the caller then takes the eight codes one by one.  (A quad or pair that fails
     // only because its codes are too long TOGETHER is retried one form down first.)
-    template <bool VALUES>
-    CLX_HD bool fast_group_t(int32_t (&e)[8]) {
+    CLX_HD bool fast_group(int32_t (&e)[8]) {
         if (!io.prefetch_group(o)) io.ensure(o);  // the ring had fallen behind (a dense stretch): refill it, blocking
         const uint32_t o0 = o, w0 = W0, w1 = W1, w2 = W2;
-        bool bad = codes8_by_cap<VALUES>(e);
+        bool bad = ncap == 2 ? codes8<2, true>(e) : codes8<1, true>(e);
         if (bad && ncap > 1) {  // once more, one code per refill: needs the window back
             o = o0; W0 = w0; W1 = w1; W2 = w2;
             io.seek_next((o0 >> 5) + 3);
-            bad = codes8<1, VALUES>(e);
+            bad = codes8<1, true>(e);
         }
         if (bad) { o = o0; n_fast = 0; wvalid = false; return false; }
         n_left -= 8;
         n_fast--;
         return true;
     }
-    CLX_HD bool fast_group(int32_t (&e)[8]) { return fast_group_t<true>(e); }
-    CLX_HD bool skip_group() {  // the same eight codes, positions only
+    // ---- a run of `groups` groups of eight codes, positions only (the index lane's walk) ----
+    // Preconditions: the window is seated, 1 <= groups <= MAXG, groups <= n_fast (the run stays inside the
+    // partition), NC <= ncap.  One ring refill covers the whole run.  Groups are committed as they go: a group that
+    // does not fit — a pair longer than 32 bits together, a code longer than the window — ends the run at its first
+    // code, with the fast path closed and false returned, and the caller takes it from there (the window is re-seated
+    // at the cursor, so nothing is saved here and nothing is retried).  Afterwards cursor, n_left and n_fast are what
+    // `groups` single-group runs would have left.
+    template <int NC, uint32_t MAXG>
+    CLX_HD bool skip_run(uint32_t groups) {
+        // a group is at most 8 * 16 bits = 1 quad long with two codes per 32-bit window, 8 * 32 bits with one
+        io.prefetch_run(o, MAXG * (NC == 2 ? 1u : 2u));
         int32_t unused[8];
-        return fast_group_t<false>(unused);
+        uint32_t g = 0, o0 = o;
+        bool bad = false;
+#pragma unroll
+        for (; g < MAXG; g++) {
+            o0 = o;
+            bad = codes8<NC, false>(unused);
+            if (bad || g + 1 == groups) break;  // one exit test per group
+        }
+        g += bad ? 0u : 1u;  // groups taken
+        n_left -= 8u * g;
+        if (bad) { o = o0; n_fast = 0; wvalid = false; return false; }
+        n_fast -= groups;
+        return true;
     }
     // The same group SPECULATIVELY and branch-free, whatever the lane's state (every memory access it makes is
     // safe in any state): the caller learns afterwards whether the residuals are real.  This lets the caller put
@@ -380,10 +398,23 @@ struct IndexLane {
     CLX_HD void fail() { rc.fail(); mode = SEQ_DONE; }
     CLX_HD bool ok() const { return rc.ok; }
     CLX_HD bool done() const { return mode == SEQ_DONE; }
+    static constexpr uint32_t RUN = 4;  // at most this many groups of eight codes per run
+    // slow_budget of a lane whose group of pairs did not fit: its next slow step retries the group one code per
+    // window refill before it takes the codes one by one
+    static constexpr uint32_t RETRY_SINGLES = 9;
     CLX_HD bool fast_ready() const { return mode == SEQ_RUN && rc.n_fast != 0; }
-    CLX_HD void fast_group() {
-        if (!rc.skip_group()) { slow_budget = 8; return; }
-        if (rc.n_left == 0 && rc.ok) {
+    // A run of min(n_fast, cap) groups of eight codes (cap <= RUN), two codes per window refill where the
+    // partition's Rice parameter allows; then the next partition if this one has ended.  A partition's last groups
+    // are a shorter run, so that a warp whose lanes cross partition boundaries at different times stays in its
+    // tight loop.
+    CLX_HD void run(uint32_t cap = RUN) {
+        const uint32_t groups = rc.n_fast < cap ? rc.n_fast : cap;
+        const bool good = rc.ncap == 2 ? rc.template skip_run<2, RUN>(groups) : rc.template skip_run<1, RUN>(groups);
+        slow_budget = good ? slow_budget : rc.ncap == 2 ? RETRY_SINGLES : 8u;
+        if (good) after_group();
+    }
+    CLX_HD void after_group() {
+        if (rc.n_left == 0) {
             if (rc.parts_left == 0) end_of_body();
             else if (rc.wvalid) {
                 // The next partition's parameter straight from the seated window, so that a warp whose lanes cross
@@ -520,6 +551,11 @@ struct IndexLane {
             }
             if (!rc.ok) { fail(); return; }
             if (rc.n_fast != 0 && slow_budget == 0) return;  // next step: a fast group
+        }
+        if (slow_budget == RETRY_SINGLES) {  // (n_left >= 8: the group that failed is still ahead)
+            rc.window_seek();
+            if (rc.template skip_run<1, 1>(1)) { slow_budget = 0; after_group(); return; }
+            slow_budget = 8;  // a code longer than the window: one by one
         }
         if (slow_budget == 0 && rc.n_left >= 8) {
             if (!rc.wvalid) rc.window_seek();

@@ -30,9 +30,62 @@ struct HostIO {
     void ensure(uint32_t) {}
     void ensure_near(uint32_t) {}
     bool prefetch_group(uint32_t) { return true; }
+    void prefetch_run(uint32_t, uint32_t) {}
 };
 
+// The index lane's walk as index_frames_kernel schedules it: runs of up to `run_groups` (<= IndexLane::RUN) groups,
+// fewer at a partition's end, slow steps for everything else.  stats (optional): [0] runs of run_groups groups,
+// [1] shorter runs, [2 + j] runs that ended at their group j on a code that did not fit the window (j < 8).
+// False: run-away.
+bool walk_index(clx::IndexLane<HostIO>& I, uint32_t run_groups, uint64_t* stats) {
+    uint64_t guard = 0;
+    while (!I.done()) {
+        if (I.fast_ready()) {
+            const uint32_t g = I.rc.n_fast < run_groups ? I.rc.n_fast : run_groups;
+            const uint32_t n0 = I.rc.n_left;
+            I.run(run_groups);
+            if (stats) {
+                stats[g == run_groups ? 0 : 1]++;
+                if (I.mode == clx::SEQ_RUN && !I.rc.wvalid) {  // the run ended early (still in its partition)
+                    const uint32_t done = (n0 - I.rc.n_left) / 8;
+                    if (done < 8) stats[2 + done]++;
+                }
+            }
+        } else {
+            I.slow_step();
+        }
+        if (++guard > (1ull << 32)) return false;
+    }
+    return true;
+}
+
 }  // namespace
+
+// The index lane alone, with runs of `run_groups` groups: per subframe slot (n * CH of them, CH = the channel count
+// rounded up to a power of two) the bit at which its residual starts, 0xffffffff for slots the frame does not
+// use; per frame 0 (walked) or -2 (declined).  stats as walk_index.  Returns CH, or -1 on a run-away.
+extern "C" int seq_host_index(const uint8_t* bytes, uint64_t nbytes, const clx_frame_desc* descs, uint32_t n,
+                              uint32_t run_groups, uint32_t* res_bit, int32_t* status, uint64_t* stats) {
+    uint32_t max_ch = 1;
+    for (uint32_t i = 0; i < n; i++)
+        if (descs[i].n_channels > max_ch) max_ch = descs[i].n_channels;
+    uint32_t CH = 1;
+    while (CH < max_ch) CH <<= 1;
+    std::vector<clx::SeqParams> params(CH);
+    for (uint32_t f = 0; f < n; f++) {
+        const clx_frame_desc& d = descs[f];
+        const uint64_t aligned = d.byte_offset & ~15ull;
+        clx::IndexLane<HostIO> I;
+        I.rc.io.base = bytes + aligned;
+        I.rc.io.avail = nbytes - aligned;
+        for (auto& p : params) p.res_bit = 0xffffffffu;
+        I.init(d, params.data(), CH);
+        if (!walk_index(I, run_groups, stats)) return -1;
+        status[f] = I.ok() ? 0 : -2;
+        for (uint32_t c = 0; c < CH; c++) res_bit[(size_t)f * CH + c] = c < d.n_channels ? params[c].res_bit : 0xffffffffu;
+    }
+    return (int)CH;
+}
 
 // head_pad: extra groups of eight samples taken one by one before the grouped part starts, as happens
 // to a lane whose warp holds a subframe of a higher order; odd values also make the speculative group take one
@@ -56,12 +109,7 @@ extern "C" int seq_host_decode(const uint8_t* bytes, uint64_t nbytes, const clx_
         I.rc.io.base = bytes + aligned;
         I.rc.io.avail = nbytes - aligned;
         I.init(d, params.data() + (size_t)f * CH, CH);
-        uint64_t guard = 0;
-        while (!I.done()) {
-            if (I.fast_ready()) I.fast_group();
-            else I.slow_step();
-            if (++guard > (1ull << 32)) return -1;  // run-away
-        }
+        if (!walk_index(I, clx::IndexLane<HostIO>::RUN, nullptr)) return -1;  // run-away
         if (!I.ok()) continue;
         // ---- one subframe lane per channel ----
         const uint32_t bs = d.block_size;
